@@ -370,6 +370,13 @@ def suggest_e2e_leg(device_index, reps=3):
 # --------------------------------------------------------------------------------------------------
 # GPU arm
 # --------------------------------------------------------------------------------------------------
+def dump_outputs(out_dir, arrays):
+  """Writes each array as out_dir/<name>.npy (float64), so that two builds can be compared output for output."""
+  os.makedirs(out_dir, exist_ok=True)
+  for name, a in arrays.items():
+    np.save(os.path.join(out_dir, f'{name}.npy'), np.asarray(a, dtype=np.float64))
+
+
 def run_gpu(args):
   import torch
   from vizier_b200 import gp
@@ -440,6 +447,13 @@ def run_gpu(args):
     step_ev[i + 1].record(stream)
   drain(args.steps)
   torch.cuda.synchronize()
+  if args.dump_outputs:
+    # read now: the legs below overwrite the score buffers
+    w_idx, w_val, w_x = state['winner']
+    dumped = {'scores' if world == 1 else f'scores_rank{rank}': outs[(args.steps - 1) % 2].cpu().numpy()}
+    if rank == 0:
+      dumped.update(winner_index=w_idx.astype(np.float64), winner_score=w_val, winner_x=w_x)
+    dump_outputs(args.dump_outputs, dumped)
   if dist is not None:
     dist.barrier()
   launches = dev.launch_count - l0
@@ -629,7 +643,15 @@ def main():
   ap.add_argument('--no-suggest', action='store_true', help='skip the suggest() end-to-end leg (N=1)')
   ap.add_argument('--no-cpu', action='store_true',
                   help='skip the cpu_baseline leg and everything that spawns processes (runs under ncu)')
+  ap.add_argument('--dump-outputs', metavar='DIR',
+                  help='after the timed steps, write what the last one returned to DIR/<name>.npy (float64): '
+                       'scores (this rank\'s candidate scores; scores_rank<r> when there are several ranks), '
+                       'winner_index, winner_score and winner_x (the merged global arg-max)')
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.dump_outputs and args.impl != 'b200':
+    ap.error('--dump-outputs writes the outputs of the GPU path (--impl b200)')
   args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
   if args.impl == 'reference':
     run_reference(args)
